@@ -78,7 +78,13 @@ def parse():
     ap.add_argument("--dense-batch", type=int, default=1024)
     ap.add_argument("--callers-seconds", type=float, default=1.0)
     ap.add_argument("--recipe", default="embedding", choices=sorted(RECIPES))
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write rank 0's results of the last timed step (ids, scores, counts) to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or a.workload != "hnsw"):
+        ap.error("--dump-outputs applies to the default workload (--impl ours --workload hnsw)")
     global KIND, SIGMA
     KIND, SIGMA = RECIPES[a.recipe]["kind"], RECIPES[a.recipe]["sigma"]
     return a
@@ -265,6 +271,51 @@ def recall_at_k(found, truth):
     return hit / float(truth.size)
 
 
+QUERY_RING = 16
+
+
+def step_sets(n_sets, make):
+    """The query set of each of n_sets steps (warm-up included), make(set index) called at most QUERY_RING times so that
+    memory does not grow with --steps.  Step 0 keeps set 0 (the recall and parity checks read it) and the last
+    QUERY_RING - 1 steps keep their own sets; the steps in between cycle through those, so consecutive steps never share a
+    set and up to QUERY_RING steps every step has a set of its own."""
+    r = QUERY_RING - 1
+    order = [0] + [s + (n_sets - 1 - s) // r * r for s in range(1, n_sets)]
+    made = {}
+    for i in order:
+        if i not in made:
+            made[i] = make(i)
+    return [made[i] for i in order]
+
+
+def map_sets(sets, f):
+    """[f(q) for q in sets], f applied once per distinct set: steps that share a set share its copy."""
+    done = {}
+    for q in sets:
+        if id(q) not in done:
+            done[id(q)] = f(q)
+    return [done[id(q)] for q in sets]
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, ids, scores, counts):
+    """Writes one step's answer as the caller receives it: ids [B,k] as float64 (exact below 2^53), scores [B,k] and
+    counts [B] as float32.  Above DUMP_BYTES a fixed seeded sample of query rows stands for the batch; the sampled row
+    indices are written as sample_rows.npy."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    rows = np.arange(len(counts))
+    row_bytes = ids.shape[1] * 8 + scores.shape[1] * 4 + 4 + 8
+    if len(rows) * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(SEED).choice(len(rows), (DUMP_BYTES - 4096) // row_bytes, replace=False))
+        np.save(out / "sample_rows.npy", rows.astype(np.float64))
+    np.save(out / "ids.npy", ids[rows].astype(np.float64))
+    np.save(out / "scores.npy", scores[rows].astype(np.float32))
+    np.save(out / "counts.npy", counts[rows].astype(np.float32))
+
+
 # ------------------------------------------------------------------------------------------------------------------
 # Sub-results carried by the default line (driver-visible evidence for every BASELINE config, VERDICT r1 item 1c)
 REF_PREFILTER_SHAPES = [("prefilter-100", 0, 100), ("prefilter-1000", 100, 1_000), ("prefilter-10000", 1_100, 10_000),
@@ -284,7 +335,7 @@ def _timed_device(torch, dev, steps, warmup, fn):
     return e0.elapsed_time(e1)
 
 
-def measure_prefilter(hx, torch, ix, args, dev, stream, n, dim, ora=None, label_steps=None):
+def measure_prefilter(hx, torch, ix, args, dev, stream, n, dim, ora=None):
     """Config C3 on an index whose ids are 0..n-1: (a) the graph-label filter — 100 queries per step, query b restricted to
     {id : id mod 100 == b} (1 % each: one step streams every row once), (b) the reference's own prefilter shapes — one
     contiguous id range of 100 / 1k / 10k / 100k candidates shared by 64 queries.  Exact scan (k_scan + k_select);
@@ -292,11 +343,11 @@ def measure_prefilter(hx, torch, ix, args, dev, stream, n, dim, ora=None, label_
     import ctypes as C
     k, sel = K, 100
     B = sel
-    steps = label_steps or args.steps
+    steps = args.steps
     hbm_peak, peak_src = measured_peaks()
     n_sets = steps + args.warmup
-    qsets = [ix.generate_queries(SEED, B, first_query=20_000_000 + s * B, n_centroids=N_CENTROIDS, sigma=SIGMA, kind=KIND)
-             for s in range(n_sets)]
+    qsets = step_sets(n_sets, lambda s: ix.generate_queries(SEED, B, first_query=20_000_000 + s * B, n_centroids=N_CENTROIDS,
+                                                            sigma=SIGMA, kind=KIND))
     cand_lists = [np.arange(b, n, sel, dtype=np.uint64) for b in range(B)]
     cand_ids = np.concatenate(cand_lists)
     offs = np.zeros(B + 1, dtype=np.uint64)
@@ -305,7 +356,7 @@ def measure_prefilter(hx, torch, ix, args, dev, stream, n, dim, ora=None, label_
     total = int(offs[-1])
     d_slots = torch.from_numpy(cand_ids.astype(np.uint32).view(np.int32)).to(dev)      # ids == slots here (first_id 0)
     d_offs = torch.from_numpy(offs.view(np.int64)).to(dev)
-    d_q = [torch.from_numpy(q).to(dev) for q in qsets]
+    d_q = map_sets(qsets, lambda q: torch.from_numpy(q).to(dev))
     o_ids = torch.zeros((B, k), dtype=torch.int64, device=dev)
     o_sc = torch.zeros((B, k), dtype=torch.float32, device=dev)
     o_cnt = torch.zeros((B,), dtype=torch.int32, device=dev)
@@ -332,7 +383,7 @@ def measure_prefilter(hx, torch, ix, args, dev, stream, n, dim, ora=None, label_
     last_q = qsets[args.warmup + steps - 1]
     L = hx.load_library()
     cp = params._c()
-    h_q = [torch.from_numpy(q).pin_memory() for q in qsets]
+    h_q = map_sets(qsets, lambda q: torch.from_numpy(q).pin_memory())
     h_c = torch.from_numpy(cand_ids.view(np.int64)).pin_memory()
     h_o = torch.from_numpy(offs.view(np.int64)).pin_memory()
     h_ids = torch.zeros((B, k), dtype=torch.int64).pin_memory()
@@ -577,10 +628,11 @@ def measure_dense(hx, torch, args, world, rank, local_rank, dev, stream, uid):
     peaks = json.loads((ROOT / "MEASURED_PEAKS.json").read_text()) if (ROOT / "MEASURED_PEAKS.json").exists() else {}
     tf_peak = float(peaks.get("bf16_tflops", 1590.0))
     steps = args.steps
-    qsets = [ix.generate_queries(SEED, B, first_query=30_000_000 + s * B, n_centroids=N_CENTROIDS, sigma=SIGMA, kind=KIND)
-             for s in range(steps + args.warmup)]          # every rank answers the SAME queries
+    qsets = step_sets(steps + args.warmup,          # every rank answers the SAME queries
+                      lambda s: ix.generate_queries(SEED, B, first_query=30_000_000 + s * B, n_centroids=N_CENTROIDS,
+                                                    sigma=SIGMA, kind=KIND))
     params = hx.SearchParams.strict(k)
-    d_q = [torch.from_numpy(q).to(dev) for q in qsets]
+    d_q = map_sets(qsets, lambda q: torch.from_numpy(q).to(dev))
     o_ids = torch.zeros((B, k), dtype=torch.int64, device=dev)
     o_sc = torch.zeros((B, k), dtype=torch.float32, device=dev)
     o_cnt = torch.zeros((B,), dtype=torch.int32, device=dev)
@@ -596,7 +648,7 @@ def measure_dense(hx, torch, args, world, rank, local_rank, dev, stream, uid):
     ms_total = float(t.item())
     dev_ids = o_ids.cpu().numpy().view(np.uint64).copy()
     # e2e: host buffers through hx_search_sharded (H2D queries, D2H merged results, one stream sync)
-    h_q = [torch.from_numpy(q).pin_memory().numpy() for q in qsets]
+    h_q = map_sets(qsets, lambda q: torch.from_numpy(q).pin_memory().numpy())
     for s in range(args.warmup):
         g.search(sh.DENSE, h_q[s], params, k)
     if world > 1:
@@ -684,13 +736,13 @@ def measure_d1536(hx, torch, args, local_rank, dev, stream):
     a2.dim, a2.metric, a2.n = 1536, "euclidean", args.d1536_rows
     n, dim, k = a2.n, a2.dim, K
     Q = 16384
-    steps = max(2, min(args.steps, 5))
+    steps = args.steps
     ix, setup = build_index(hx, a2, local_rank, 0, n)
     hbm_peak, peak_src = measured_peaks()
-    qsets = [ix.generate_queries(SEED, Q, first_query=40_000_000 + s * Q, n_centroids=N_CENTROIDS, sigma=SIGMA, kind=KIND)
-             for s in range(steps + args.warmup)]
+    qsets = step_sets(steps + args.warmup, lambda s: ix.generate_queries(SEED, Q, first_query=40_000_000 + s * Q,
+                                                                         n_centroids=N_CENTROIDS, sigma=SIGMA, kind=KIND))
     params = hx.SearchParams.strict(k, EF)
-    d_q = [torch.from_numpy(q).to(dev) for q in qsets]
+    d_q = map_sets(qsets, lambda q: torch.from_numpy(q).to(dev))
     o_ids = torch.zeros((Q, k), dtype=torch.int64, device=dev)
     o_sc = torch.zeros((Q, k), dtype=torch.float32, device=dev)
     o_cnt = torch.zeros((Q,), dtype=torch.int32, device=dev)
@@ -724,7 +776,7 @@ def measure_d1536(hx, torch, args, local_rank, dev, stream):
     import ctypes as C
     L = hx.load_library()
     cp = params._c()
-    h_q = [torch.from_numpy(qsets[args.warmup + s]).pin_memory() for s in range(steps)]
+    h_q = map_sets(qsets[args.warmup:], lambda q: torch.from_numpy(q).pin_memory())
     h_ids = torch.zeros((Q, k), dtype=torch.int64).pin_memory()
     h_sc = torch.zeros((Q, k), dtype=torch.float32).pin_memory()
     h_cnt = torch.zeros((Q,), dtype=torch.int32).pin_memory()
@@ -766,7 +818,7 @@ def measure_d1536(hx, torch, args, local_rank, dev, stream):
                                "ids_identical_to_device": bool(ci.tolist() == first_ids[:ns].tolist()),
                                "scores_identical_to_device": bool(cs.tobytes() == first_sc[:ns].tobytes()),
                                "mirror_s": round(mirror_s, 1)}
-        pf = measure_prefilter(hx, torch, ix, a2, dev, stream, n, dim, ora=ora, label_steps=2)
+        pf = measure_prefilter(hx, torch, ix, a2, dev, stream, n, dim, ora=ora)
         out["prefilter_reference_shapes"] = pf["reference_shapes"]
         out["prefilter_label_sets"] = {"value": pf["value"], "roofline_frac": pf["roofline"]["frac"],
                                        "bit_exact_vs_oracle": pf.get("cpu_baseline", {}).get("bit_exact_vs_device")}
@@ -801,11 +853,11 @@ def run_ours(args):
     # ---- setup (untimed): corpus on the device, graph built on the device ---------------------------------------
     ix, setup = build_index(hx, args, local_rank, 0, n)
     n_sets = args.steps + args.warmup
-    # distinct queries every step and every rank (nothing can be answered from a previous step's cache lines)
-    qsets = [ix.generate_queries(SEED, Q, first_query=(rank * n_sets + s) * Q, n_centroids=N_CENTROIDS, sigma=SIGMA, kind=KIND)
-             for s in range(n_sets)]
+    # distinct queries every rank and in consecutive steps (nothing can be answered from a previous step's cache lines)
+    qsets = step_sets(n_sets, lambda s: ix.generate_queries(SEED, Q, first_query=(rank * n_sets + s) * Q,
+                                                            n_centroids=N_CENTROIDS, sigma=SIGMA, kind=KIND))
     params = hx.SearchParams.strict(k, EF)
-    d_q = [torch.from_numpy(q).to(dev) for q in qsets]
+    d_q = map_sets(qsets, lambda q: torch.from_numpy(q).to(dev))
     o_ids = torch.zeros((Q, k), dtype=torch.int64, device=dev)
     o_sc = torch.zeros((Q, k), dtype=torch.float32, device=dev)
     o_cnt = torch.zeros((Q,), dtype=torch.int32, device=dev)
@@ -838,6 +890,9 @@ def run_ours(args):
     e1.record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    last_step = None
+    if args.dump_outputs and rank == 0:       # the last timed step's answer, copied after the timed region closed
+        last_step = (o_ids.cpu().numpy().view(np.uint64).copy(), o_sc.cpu().numpy().copy(), o_cnt.cpu().numpy().copy())
     ms_total = e0.elapsed_time(e1)
     kernel_ms_total, kernel_launches = ix.last_kernel_ms()
     dev_flags, dev_flag_status = ix.device_flags(stream)   # error flags ORed over the timed launches (ADVICE r1): must be 0
@@ -865,7 +920,7 @@ def run_ours(args):
     achieved = bytes_per_launch / (kernel_ms * 1e-3) / 1e9 if kernel_ms > 0 else 0.0
 
     # ---- e2e: reference-facing C-ABI call with host (pinned) buffers -------------------------------------------------
-    h_q = [torch.from_numpy(q).pin_memory() for q in qsets]
+    h_q = map_sets(qsets, lambda q: torch.from_numpy(q).pin_memory())
     h_ids = torch.zeros((Q, k), dtype=torch.int64).pin_memory()
     h_sc = torch.zeros((Q, k), dtype=torch.float32).pin_memory()
     h_cnt = torch.zeros((Q,), dtype=torch.int32).pin_memory()
@@ -989,8 +1044,9 @@ def run_ours(args):
         sx, s_setup = build_index(hx, args, local_rank, lo, hi - lo)
         grp = sh.ShardGroup(sx, world, rank, uid)
         # every rank searches the SAME queries (rank 0's sets) against its shard
-        sq = [ix.generate_queries(SEED, Q, first_query=s * Q, n_centroids=N_CENTROIDS, sigma=SIGMA, kind=KIND) for s in range(n_sets)]
-        d_sq = [torch.from_numpy(q).to(dev) for q in sq]
+        sq = step_sets(n_sets, lambda s: ix.generate_queries(SEED, Q, first_query=s * Q, n_centroids=N_CENTROIDS, sigma=SIGMA,
+                                                             kind=KIND))
+        d_sq = map_sets(sq, lambda q: torch.from_numpy(q).to(dev))
         truth_s = exact_topk_device(hx, torch, ix, sq[0][:rq], n, 0, k)
         step_device(0)   # the unsharded index on the same queries: the recall the shards have to match
         ix.search_device(d_sq[0].data_ptr(), Q, params, o_ids.data_ptr(), o_sc.data_ptr(), o_cnt.data_ptr(), stream)
@@ -1035,7 +1091,7 @@ def run_ours(args):
         barrier()
         f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         f0.record()
-        for s in range(min(args.steps, 4)):
+        for s in range(args.steps):
             run_sharded(args.warmup + s, p_full)
         f1.record()
         barrier()
@@ -1045,7 +1101,7 @@ def run_ours(args):
         sharded = {"value": round(args.steps * Q / (float(ts.item()) / 1e3), 1), "unit": "queries/s",
                    "recall_at_10": round(s_recall, 4), "unsharded_recall_at_10_same_queries": round(target, 4),
                    "ef_per_shard": chosen, "k_per_shard": k, "iso_recall_tuning": tuning,
-                   "value_at_unsharded_ef": round(min(args.steps, 4) * Q / (float(tf_.item()) / 1e3), 1),
+                   "value_at_unsharded_ef": round(args.steps * Q / (float(tf_.item()) / 1e3), 1),
                    "shard_vectors": hi - lo,
                    "api": "hx_search_sharded_device (C ABI): local search into the send block, ncclAllGather, merge kernel",
                    "collective": f"1 x ncclAllGather of {blk} B per rank per step (issued by libhelix_b200 via dlopen'ed NCCL)",
@@ -1136,6 +1192,8 @@ def run_ours(args):
     ix.close()
     if rank == 0 and world == 1 and not args.no_subresults and not args.no_d1536:
         line["euclid_d1536"] = measure_d1536(hx, torch, args, local_rank, dev, stream)
+    if last_step is not None:
+        dump_outputs(args.dump_outputs, *last_step)
     if rank == 0:
         print(json.dumps(line), flush=True)
         if parity is not None and not (parity["ids_identical_to_device"] and parity["scores_identical_to_device"]):
